@@ -17,6 +17,15 @@ TIP3P waters (99,999 atoms, fp32).  Rank 0 prints ONE JSON line:
              timed region) against the measured HBM peak (MEASURED_PEAKS.json)
   cpu_baseline  the oracle port of the reference's all-pairs PyTorch-CPU path timed on
              this box's host cores on a bounded sample (smaller box, O(N^2) scaled)
+
+--dump-outputs DIR (one GPU) writes what the last timed step left to a caller of Integrator.step, as
+DIR/<name>.npy: positions, velocities, forces (replicas, atoms, 3) float32 and the per-replica
+kinetic_energy, potential_energy and temperature.  So that the same arguments give the same inputs on
+every run and two builds can be compared output for output, the warm-up then runs a fixed number of
+steps (not "at least 0.6 s") and the relaxation of the water boxes runs on the full Verlet rows, whose
+force sums have a fixed order.  The warm-up and the timed steps stay on the default path: where that is
+the cluster path, whose force sums depend on the order of arrival, two runs differ by rounding that the
+dynamics amplify with every step, so per-atom arrays are comparable over short runs only.
 """
 import argparse
 import json
@@ -313,6 +322,8 @@ def gpu_arm(args):
     local = int(os.environ.get("LOCAL_RANK", "0"))
     wl = args.workload
     replicated = wl in ("thrombin16", "water291")
+    if args.dump_outputs and world > 1:
+        raise SystemExit("--dump-outputs runs with one GPU")
     if world > 1:
         # (NCCL's own log, if NCCL_DEBUG is set, goes to stderr / NCCL_DEBUG_FILE; rank 0 prints the JSON line last)
         if not dist.is_initialized():  # (tests/test_domain_host.py brings its own gloo group)
@@ -341,6 +352,11 @@ def gpu_arm(args):
     system.set_box(boxd)
     torch.manual_seed(1 + rank)
     system.set_velocities(maxwell_boltzmann(par.masses, TEMPERATURE, nrep))
+    # --dump-outputs: the relaxation runs on the full Verlet rows, whose force sums have a fixed order, so that every run
+    # enters the warm-up from the same state (the cluster path adds forces in arrival order, and MD amplifies the last bits)
+    relax_env = {"TMD_B200_CLUSTER": "0"} if args.dump_outputs and needs_eq else {}
+    env_before = {k: os.environ.get(k) for k in relax_env}
+    os.environ.update(relax_env)
     forces = Forces(par, terms=terms, **cfg)
     forces.compute(system.pos, system.box, system.forces)
 
@@ -351,7 +367,12 @@ def gpu_arm(args):
         for _ in range(args.equil // 100):
             eq.step(niter=100)
             equil_done += 100
-        if equil_done:
+        for k, v in env_before.items():  # the warm-up and the timed steps run the default path
+            if v is None:
+                os.environ.pop(k)
+            else:
+                os.environ[k] = v
+        if equil_done or relax_env:
             # A lattice start can be refused by the cluster lists (its 4-atom clusters are too long for a small box) and the
             # context then waits >= 1000 force calls before it tries them again: the melted configuration gets a fresh one.
             forces = Forces(par, terms=terms, **cfg)
@@ -362,7 +383,8 @@ def gpu_arm(args):
     chunk = 50 if n > 20000 else 500
     nwarm = max(3, args.warmup, chunk if world == 1 else 4 * chunk)
     done = 0
-    while done < nwarm or (world == 1 and time.perf_counter() - t_w < 0.6):  # >= 0.6 s under load for the sampler
+    # >= 0.6 s under load for the sampler; a fixed step count when the outputs are dumped (a reproducible start)
+    while done < nwarm or (world == 1 and not args.dump_outputs and time.perf_counter() - t_w < 0.6):
         ekin, pot, T = integ.step(niter=chunk)
         done += chunk
 
@@ -377,6 +399,8 @@ def gpu_arm(args):
     ekin, pot, T = integ.step(niter=args.steps)
     ev1.record()
     torch.cuda.synchronize()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, system, ekin, pot, T)
     import ctypes as C
 
     # The timed steps are replays of a captured step (one graph launch per step); a kernel inside a replay cannot be
@@ -546,10 +570,33 @@ def gpu_arm(args):
     print(json.dumps(line), flush=True)
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, system, ekin, pot, T):
+    """The state and the return values of the last timed Integrator.step call, one .npy file each."""
+    import numpy as np
+
+    arrays = {
+        "positions": system.pos.detach().cpu().numpy(),
+        "velocities": system.vel.detach().cpu().numpy(),
+        "forces": system.forces.detach().cpu().numpy(),
+        "kinetic_energy": np.asarray(ekin, np.float32),
+        "potential_energy": np.asarray(pot, np.float64),
+        "temperature": np.asarray(T, np.float32),
+    }
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit(f"--dump-outputs: {total} bytes of outputs exceed {DUMP_LIMIT_BYTES}")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=3000)
+    ap.add_argument("--steps", type=int, default=3000, help="timed MD steps (>= 1)")
     ap.add_argument("--warmup", type=int, default=200)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--equil", type=int, default=600, help="relaxation steps before warm-up (lattice start)")
@@ -557,7 +604,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--workload", default="water100k", choices=sorted(WORKLOADS),
                     help="water100k is BASELINE.json's headline; the others are its configs 2, 3, 5 and the 9,999-atom box both arms can run")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step to DIR/<name>.npy (see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     if args.impl == "reference":
         return reference_arm(args)
     return gpu_arm(args)

@@ -1,18 +1,16 @@
 """The AMBER prmtop / NAMD coordinate readers (SURVEY.md section 8f-2) against the reference's STORED
-known answers for tests/data/prod_alanine_dipeptide_amber, through the CPU oracle.  Needs the
-reference checkout for the input files (skipped where it is absent, e.g. on the GPU box; the GPU
-parity tests use the parsed parameters committed in tests/golden/ala2_*.npz instead)."""
+known answers for its tests/data/prod_alanine_dipeptide_amber, through the CPU oracle.  The input files
+are the reference's, copied into tests/golden/data/ (copy_reference_data.py); the GPU parity tests use
+the parsed parameters committed in tests/golden/ala2_*.npz."""
 import os
 
 import numpy as np
-import pytest
 import torch
 
-from conftest import load_golden
+from conftest import GOLDEN, load_golden
 from oracle import refmd
 
-ALA = "/root/reference/tests/data/prod_alanine_dipeptide_amber"
-pytestmark = pytest.mark.skipif(not os.path.isdir(ALA), reason="reference data files not present")
+ALA = os.path.join(GOLDEN, "data", "prod_alanine_dipeptide_amber")
 TERMS = ["bonds", "angles", "dihedrals", "impropers", "1-4", "electrostatics", "lj"]
 
 

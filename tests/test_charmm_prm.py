@@ -1,7 +1,8 @@
 """CHARMM .prm reader (torchmd_b200/charmm.py CharmmPrmForceField) and the parameter tables built from it, against the
 UNMODIFIED reference's Parameters on the reference's own small CHARMM fixtures.  The goldens (tests/golden/charmm_*.npz,
-make_golden_charmm.py) hold the reference's tables and its Forces.compute results; the reader tests need the reference
-checkout for the input files and are skipped where it is absent."""
+make_golden_charmm.py) hold the reference's tables and its Forces.compute results; the reader tests parse the reference's
+input files, copied into tests/golden/data/ (copy_reference_data.py: the large parameters.prm files keep only the entries
+of each fixture's own atom types)."""
 import glob
 import os
 
@@ -9,12 +10,11 @@ import numpy as np
 import pytest
 import torch
 
-from conftest import golden_cfg, golden_system_tensors, load_golden, params_from_golden
+from conftest import GOLDEN, golden_cfg, golden_system_tensors, load_golden, params_from_golden
 from oracle import refmd
 
-DATA = "/root/reference/tests/data"
+DATA = os.path.join(GOLDEN, "data")
 CASES = ["1water", "2ions", "3ions", "1dihedral", "singledihedral", "4dihedrals", "benzamidine", "2watersperiodic", "sodiumperiodic", "waterbox"]
-needs_files = pytest.mark.skipif(not os.path.isdir(DATA), reason="reference data files not present")
 
 
 def files(name):
@@ -22,7 +22,6 @@ def files(name):
     return tuple(glob.glob(os.path.join(folder, e))[0] for e in ("*.psf", "*.pdb", "*.prm"))
 
 
-@needs_files
 @pytest.mark.parametrize("name", CASES)
 def test_tables_from_the_prm_reader_equal_the_reference_parameters(name):
     """yaml_parameters(mol, CharmmPrmForceField) -- the package's own table builder -- reproduces what the reference's
@@ -47,7 +46,6 @@ def test_tables_from_the_prm_reader_equal_the_reference_parameters(name):
                 assert torch.equal(a[key], b[key]), (attr, key)
 
 
-@needs_files
 def test_tip3p_in_the_prm_file_is_the_tip3p_of_the_reference_yaml():
     """The one cross-check the reference's own files offer: its CHARMM water parameters and its YAML water force field
     (tests/water) describe the same model."""
@@ -55,7 +53,7 @@ def test_tip3p_in_the_prm_file_is_the_tip3p_of_the_reference_yaml():
     from torchmd_b200.ff_yaml import YamlForceField
 
     ff = charmm.CharmmPrmForceField(files("1water")[2])
-    y = YamlForceField("/root/reference/tests/water/water_forcefield.yaml")
+    y = YamlForceField(os.path.join(DATA, "water", "water_forcefield.yaml"))
     assert ff.get_bond("OT", "HT") == tuple(y.get_bond("OT", "HT")) == ff.get_bond("HT", "OT")
     ka, ta = ff.get_angle("HT", "OT", "HT")
     ky, ty = y.get_angle("HT", "OT", "HT")

@@ -227,7 +227,7 @@ def _worker_bench(rank, world, port, out):
     bench.DEVICE_OVERRIDE, bench.MIN_DECOMPOSED_WARMUP, bench.N_WATERS = "cpu", 4, 64
     bench.CFG = dict(bench.CFG, cutoff=5.0, switch_dist=4.0)
     bench.ClockSampler = _NoSampler
-    args = argparse.Namespace(gpus=world, steps=5, warmup=3, equil=6, e2e_steps=2, no_cpu_baseline=True, impl="ours")
+    args = argparse.Namespace(gpus=world, steps=5, warmup=3, equil=6, e2e_steps=2, no_cpu_baseline=True, impl="ours", dump_outputs=None)
     buf = io.StringIO()
     with contextlib.redirect_stdout(buf), contextlib.redirect_stderr(io.StringIO()):
         domain.bench_decomposed(args, world, rank, 0, bench.workload_config(world))
@@ -319,7 +319,7 @@ def _worker_replicas(rank, world, port, out):
     torch.empty = empty
     bench.DEVICE_OVERRIDE = "cpu"
     bench.ClockSampler = _NoSampler
-    args = argparse.Namespace(gpus=world, steps=4, warmup=3, equil=0, e2e_steps=2, no_cpu_baseline=True, impl="ours", workload="water291")
+    args = argparse.Namespace(gpus=world, steps=4, warmup=3, equil=0, e2e_steps=2, no_cpu_baseline=True, impl="ours", dump_outputs=None, workload="water291")
     buf = io.StringIO()
     with contextlib.redirect_stdout(buf), contextlib.redirect_stderr(io.StringIO()):
         bench.gpu_arm(args)

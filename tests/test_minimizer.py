@@ -74,18 +74,10 @@ def test_conjugate_gradient_and_torch_lbfgs(capsys):
 
 
 def test_conjugate_gradient_follows_the_references_evaluations():
-    """Same sequence of trial points as torchmd/minimizers.py (imported from /root/reference where it exists) on an
-    anharmonic potential, where the bracket has to shrink and shift."""
-    import os
-    import sys
-
-    if not os.path.isdir("/root/reference/torchmd"):
-        pytest.skip("the reference is only present in the development container")
-    sys.path.insert(0, "/root/reference")
-    try:
-        from torchmd import minimizers as ref
-    finally:
-        sys.path.remove("/root/reference")
+    """Same sequence of trial points as the reference's torchmd/minimizers.py evaluated (stored in
+    tests/golden/minimizer_cg_trace.npz by make_golden_known_answers.py) on an anharmonic potential, where the bracket
+    has to shrink and shift."""
+    from conftest import load_golden
     from torchmd_b200 import minimizers as mine
 
     class Quartic:
@@ -98,10 +90,10 @@ def test_conjugate_gradient_follows_the_references_evaluations():
             forces.copy_(-(4 * p**3 - 6 * p + 0.5))
             return [float((p**4 - 3 * p**2 + 0.5 * p).sum())]
 
-    x0 = torch.zeros(1, 6, 3)
-    out = []
-    for mod in (ref, mine):
-        f, s = Quartic(), _system(x0, seed=3, spread=1.5)
-        out.append((mod.minimize_cg(s, f, steps=4), f.trace))
-    assert out[0][0] == out[1][0] and len(out[0][1]) == len(out[1][1]) > 20
-    assert all(torch.equal(a, b) for a, b in zip(out[0][1], out[1][1]))
+    g = load_golden("minimizer_cg_trace")
+    f, s = Quartic(), _system(torch.zeros(1, 6, 3))
+    s.pos = torch.tensor(g["start"])
+    ret = mine.minimize_cg(s, f, steps=4)
+    ref_trace = torch.tensor(g["trace"])[:, None]
+    assert ret == int(g["returned"]) and len(f.trace) == len(ref_trace) > 20
+    assert all(torch.equal(a, b) for a, b in zip(ref_trace, f.trace))

@@ -258,12 +258,8 @@ def test_multi_rank_check_script_runs_with_one_rank(hostsim, monkeypatch, capsys
     assert done.value.code == 0 and "P2P_CHECK PASS" in capsys.readouterr().out
 
 
-def test_bench_single_gpu_arm_dry_run(hostsim, monkeypatch, capsys):
-    """bench.py's own single-GPU body on a 64-water box: every library call, the profiling hooks, the host-buffer
-    entry and the JSON line's keys -- a bench that dies on a typo at round end has no number at all."""
-    import argparse
-    import json
-
+def _bench_on_the_interpreter(monkeypatch):
+    """bench.py's single-GPU arm on the host interpreter build: host events and buffers, no clock sampler, 64 waters."""
     import bench
 
     class _Event:
@@ -298,7 +294,18 @@ def test_bench_single_gpu_arm_dry_run(hostsim, monkeypatch, capsys):
     monkeypatch.setattr(bench, "CFG", dict(bench.CFG, cutoff=5.0, switch_dist=4.0))
     monkeypatch.delenv("WORLD_SIZE", raising=False)
     monkeypatch.setattr(bench, "DEVICE_OVERRIDE", "cpu")
-    args = argparse.Namespace(gpus=1, steps=6, warmup=3, equil=100, e2e_steps=3, no_cpu_baseline=True, impl="ours", workload="water100k")
+    return bench
+
+
+def test_bench_single_gpu_arm_dry_run(hostsim, monkeypatch, capsys):
+    """bench.py's own single-GPU body on a 64-water box: every library call, the profiling hooks, the host-buffer
+    entry and the JSON line's keys -- a bench that dies on a typo at round end has no number at all."""
+    import argparse
+    import json
+
+    bench = _bench_on_the_interpreter(monkeypatch)
+    args = argparse.Namespace(gpus=1, steps=6, warmup=3, equil=100, e2e_steps=3, no_cpu_baseline=True, impl="ours", workload="water100k",
+                              dump_outputs=None)
     bench.gpu_arm(args)
     line = json.loads([l for l in capsys.readouterr().out.splitlines() if l.startswith("{")][-1])
     for key in ("metric", "value", "unit", "n_gpus", "steps", "warmup", "ms_per_step", "higher_is_better", "scaling", "vs_baseline",
@@ -309,10 +316,32 @@ def test_bench_single_gpu_arm_dry_run(hostsim, monkeypatch, capsys):
     assert {"bound", "achieved", "peak", "unit", "frac", "traffic"} <= set(line["roofline"])
     # the reference's own small test systems as workloads (BASELINE configs 2 and 3), two replicas included
     for wl in ("water291", "ala2"):
-        args = argparse.Namespace(gpus=1, steps=4, warmup=3, equil=0, e2e_steps=2, no_cpu_baseline=True, impl="ours", workload=wl)
+        args = argparse.Namespace(gpus=1, steps=4, warmup=3, equil=0, e2e_steps=2, no_cpu_baseline=True, impl="ours", workload=wl,
+                                  dump_outputs=None)
         bench.gpu_arm(args)
         line = json.loads([l for l in capsys.readouterr().out.splitlines() if l.startswith("{")][-1])
         assert line["value"] > 0 and line["metric"] == bench.METRICS[wl] and line["state"]["replicas"] == (2 if wl == "water291" else 1)
+
+
+def test_bench_dump_outputs_are_reproducible(hostsim, monkeypatch, capsys, tmp_path):
+    """--dump-outputs: the same arguments write the same outputs twice, and --steps sets the number of timed steps."""
+    import argparse
+    import json
+
+    bench = _bench_on_the_interpreter(monkeypatch)
+    dumps = []
+    for run, steps in enumerate((4, 4, 5)):
+        out = tmp_path / str(run)
+        args = argparse.Namespace(gpus=1, steps=steps, warmup=3, equil=0, e2e_steps=2, no_cpu_baseline=True, impl="ours", workload="water100k",
+                                  dump_outputs=str(out))
+        bench.gpu_arm(args)
+        assert json.loads([l for l in capsys.readouterr().out.splitlines() if l.startswith("{")][-1])["steps"] == steps
+        dumps.append({p.stem: np.load(p) for p in sorted(out.glob("*.npy"))})
+    assert set(dumps[0]) == {"positions", "velocities", "forces", "kinetic_energy", "potential_energy", "temperature"}
+    assert dumps[0]["positions"].shape == (1, 192, 3) and dumps[0]["positions"].dtype == np.float32
+    assert dumps[0]["potential_energy"].shape == (1,) and dumps[0]["potential_energy"].dtype == np.float64
+    assert all(np.array_equal(dumps[0][k], dumps[1][k]) for k in dumps[0])
+    assert not np.array_equal(dumps[0]["positions"], dumps[2]["positions"])  # one more timed step, a different state
 
 
 def test_bench_reference_arm_reports_what_it_measured(monkeypatch, capsys):
@@ -393,32 +422,63 @@ def test_ab_bench_script_dry_run(hostsim, monkeypatch, capsys):
     assert abs(t[0] - t[1]) < 1e-3 * t[0] and launches[1] < launches[0], rows
 
 
-@pytest.mark.skipif(not os.path.isfile("/root/reference/tests/test_integrator.py"), reason="reference checkout not present")
-def test_the_references_own_integrator_tests_pass_against_this_package(hostsim, monkeypatch):
-    """/root/reference/tests/test_integrator.py, unmodified, with `torchmd.integrator` and `torchmd.systems` resolving
-    to this package's mirrors (SURVEY.md section 8d-vi): its eleven known-answer tests -- kinetic energy with and without
-    batches, constructor attributes, velocity-Verlet arithmetic with one and two replicas -- run through Integrator.step
-    and the integrator kernels of the (host-interpreted) library."""
-    import importlib.util
-    import sys
-    import types
+def test_the_references_own_integrator_tests_pass_against_this_package(hostsim):
+    """The scenarios of the reference's tests/test_integrator.py against what the unmodified reference computed on them
+    (tests/golden/integrator_known_answers.npz, make_golden_known_answers.py), at that file's tolerance: kinetic energy
+    with and without batches, constructor attributes, velocity-Verlet arithmetic with one and two replicas -- run through
+    Integrator.step and the integrator kernels of the (host-interpreted) library."""
+    from conftest import load_golden
+    from torchmd_b200.integrator import Integrator, kinetic_energy, kinetic_to_temp
+    from torchmd_b200.systems import System
 
-    import torchmd_b200.integrator
-    import torchmd_b200.systems
+    g = load_golden("integrator_known_answers")
+    for i in range(6):
+        batch = torch.tensor(g[f"ke{i}/batch"]) if f"ke{i}/batch" in g else None
+        out = kinetic_energy(torch.tensor(g[f"ke{i}/masses"]), torch.tensor(g[f"ke{i}/vel"]), batch=batch)
+        assert out.shape == g[f"ke{i}/out"].shape
+        np.testing.assert_allclose(out.numpy(), g[f"ke{i}/out"], rtol=1e-6)
 
-    monkeypatch.setattr(sys, "dont_write_bytecode", True)  # the reference tree is read-only
-    pkg = types.ModuleType("torchmd")
-    pkg.integrator, pkg.systems = torchmd_b200.integrator, torchmd_b200.systems
-    monkeypatch.setitem(sys.modules, "torchmd", pkg)
-    monkeypatch.setitem(sys.modules, "torchmd.integrator", torchmd_b200.integrator)
-    monkeypatch.setitem(sys.modules, "torchmd.systems", torchmd_b200.systems)
-    spec = importlib.util.spec_from_file_location("reference_test_integrator", "/root/reference/tests/test_integrator.py")
-    mod = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(mod)
-    names = [n for n in dir(mod) if n.startswith("test_")]
-    assert len(names) == 11
-    for n in names:
-        getattr(mod, n)()
+    class ConstantForces:
+        def __init__(self, forces, pot):
+            self.f, self.pot = forces, pot
+
+        def compute(self, pos, box, forces):
+            forces.copy_(self.f)
+            return self.pot
+
+    system = System(2, 1, torch.float32, "cpu")
+    system.set_masses(torch.tensor([1.0, 2.0]))
+    forces = ConstantForces(torch.zeros(1, 2, 3), 0.0)
+    plain = Integrator(system, forces, 0.001, "cpu")
+    assert plain.systems is system and plain.forces is forces and plain.device == "cpu"
+    assert plain.T is None and plain.gamma is None
+    assert plain.dt == pytest.approx(float(g["init/dt"]), rel=1e-12)
+    thermo = Integrator(system, forces, 0.001, "cpu", gamma=1.0, T=300.0)
+    assert thermo.T == 300.0 and thermo.gamma == pytest.approx(float(g["init/gamma"]), rel=1e-12)
+
+    for c in ("mock", "batches", "two_atoms", "two_replicas"):
+        pos = torch.tensor(g[c + "/pos"])
+        system = System(pos.shape[1], pos.shape[0], torch.float32, "cpu")
+        system.pos.copy_(pos)
+        system.vel.copy_(torch.tensor(g[c + "/vel"]))
+        system.set_masses(torch.tensor(g[c + "/masses"]))
+        forces = ConstantForces(torch.tensor(g[c + "/forces"]), float(g[c + "/pot"]))
+        if g[c + "/precompute"]:
+            forces.compute(system.pos, system.box, system.forces)
+        batch = torch.tensor(g[c + "/batch"]) if c + "/batch" in g else None
+        integ = Integrator(system, forces, float(g[c + "/timestep"]), "cpu", batch=batch)
+        assert integ.batch is batch and np.array_equal(integ.natoms, g[c + "/natoms"])
+        for k, n in enumerate(g[c + "/niters"]):
+            ekin, pot, temp = integ.step(niter=int(n))
+            assert isinstance(ekin, np.ndarray) and isinstance(temp, np.ndarray) and isinstance(pot, (int, float))
+            assert ekin.shape == temp.shape == g[f"{c}/ekin_{k}"].shape
+            assert pot == float(g[f"{c}/pot_{k}"])
+            np.testing.assert_allclose(system.pos.numpy(), g[f"{c}/pos_{k}"], rtol=1e-6, err_msg=c)
+            np.testing.assert_allclose(system.vel.numpy(), g[f"{c}/vel_{k}"], rtol=1e-6, err_msg=c)
+            np.testing.assert_allclose(ekin, g[f"{c}/ekin_{k}"], rtol=1e-6, err_msg=c)
+            np.testing.assert_allclose(temp, g[f"{c}/temp_{k}"], rtol=1e-6, err_msg=c)
+            np.testing.assert_allclose(ekin, kinetic_energy(system.masses, system.vel, batch=batch).numpy().flatten(), rtol=1e-6)
+            np.testing.assert_allclose(temp, kinetic_to_temp(ekin, integ.natoms), rtol=1e-6)
 
 
 def test_decomposed_integrator_replays_captured_steps(hostsim, monkeypatch):
